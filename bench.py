@@ -3,6 +3,7 @@
 (3dmpifft_opt/fftSpeed3d_c2c.cpp:126-128), per-stage t0..t3 ms, HBM-roofline fraction.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl dfft|reference] [--size 512] [--precision double]
+                    [--dump-outputs DIR]
 
 A "step" is one forward transform of the synthetic N^3 cube (BASELINE.json configs[1]: 512^3 double on
 1 GPU; the same cube sharded over N GPUs = strong scaling).  N > 1 runs one process per GPU under
@@ -27,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is cached in it
 # the CPUs this process may use, taken BEFORE any OpenMP runtime (torch's) binds the main thread to one core
 try:
     CPUS_ALLOWED = sorted(os.sched_getaffinity(0))
@@ -41,6 +43,24 @@ def pin_openmp_threads():
     step host-bound against 0.87 ms of device time, profiles/r2_final_bench_n4_hostbound.json)."""
     os.environ.setdefault("OMP_PROC_BIND", "close")
     os.environ.setdefault("OMP_PLACES", "cores")
+
+
+DUMP_BYTES = 32 << 20   # --dump-outputs: data written per run, over all ranks
+
+
+def dump_output(directory, name, out, count, ranks):
+    """Writes the first `count` elements of the complex device tensor `out` to DIR/<name>.npy as [re, im] pairs of its real
+    dtype (float64 for double, float32 for float): all of them when they fit this rank's share of DUMP_BYTES, else a fixed
+    sample at positions (k * 2654435761 + 97) mod count, k = 0, 1, ..., in increasing order -- the same on every run."""
+    import numpy as np
+    import torch
+    k = DUMP_BYTES // (ranks * out.element_size())
+    vals = out[:count]
+    if count > k:
+        pos = torch.sort((torch.arange(k, dtype=torch.int64, device=out.device) * 2654435761 + 97) % count).values
+        vals = vals.index_select(0, pos)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), torch.view_as_real(vals).cpu().numpy())
 
 
 def flops(n0, n1, n2):
@@ -330,6 +350,8 @@ def run_dfft_arm(args):
     plan.synchronize()
     barrier()
     total_ms = max_over_ranks(e0.elapsed_time(e1))
+    if args.dump_outputs:   # the last timed step's result: this rank's y-slab of the spectrum, [y_l][z][x]
+        dump_output(args.dump_outputs, f"spectrum_rank{rank}", tout, plan.out_count, P)
     ms_per_step = total_ms / args.steps
     stage = [max_over_ranks(x) for x in plan.timings()]
     passes = [max_over_ranks(x) for x in plan.pass_timings()]
@@ -503,7 +525,13 @@ def main():
     ap.add_argument("--overlap", action="store_true", help="EXPERIMENTAL: whole forward transform as one kernel, t3 overlapped behind per-part arrivals (P2P, N > 1)")
     ap.add_argument("--no-pipeline", action="store_true", help="P > 1: disable the stream-pipelined z-part forward path (t2/t3 then run after t0)")
     ap.add_argument("--fuse", action="store_true", help="force the fused L2-resident t0 kernel (default: only with the P2P exchange)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the spectrum the last step computed as DIR/spectrum_rank<r>.npy "
+                    "([re, im] pairs; a fixed sample when the whole would exceed %d MB); the input is the same on every run" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "dfft":
+        ap.error("--dump-outputs writes the outputs of the dfft arm")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_dfft_arm(args)

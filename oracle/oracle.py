@@ -271,6 +271,16 @@ class COracle:
         return float(drv), float(ab.value)
 
 
+def sampled(a, k: int) -> np.ndarray:
+    """k entries of the flattened `a` at fixed positions spread over it (all of it when k >= a.size).  The positions depend
+    only on (a.size, k) and not on numpy's random streams, so a stored sample of a large reference output can be compared
+    with the same positions of a recomputation."""
+    a = np.asarray(a).reshape(-1)
+    if k >= a.size:
+        return a.copy()
+    return a[np.unique((np.arange(k, dtype=np.int64) * 2654435761 + 97) % a.size)]   # distinct: the multiplier is a prime > a.size
+
+
 def minstd_uniform(count: int, state: int = 4242):
     """numpy restatement of heffte/heffteBenchmark/test/test_fft3d.h:19-27 input
     (std::minstd_rand(4242) -> uniform_real_distribution<double>(0,1)); returns (values, state)."""

@@ -203,23 +203,19 @@ def test_reference_driver_through_the_cxx_shim_on_a_fake_runtime(fake_lib, tmp_p
 
 
 def test_driver_stdout_surface_is_the_reference_drivers(fake_lib, tmp_path):
-    """The reference's OWN driver program (3dmpifft_opt/fftSpeed3d_c2c.cpp compiled in place against the HIP-on-CPU shim,
-    oracle/_ref/distFFT_ref, one device) and this repo's driver/distFFT.cpp (against the fake CUDA runtime) are run with the
-    same arguments: with every number replaced by '#', the reference's stdout must be, line for line and in order, a
-    subsequence of ours (ours adds lines after the report block)."""
+    """The reference's OWN driver program (3dmpifft_opt/fftSpeed3d_c2c.cpp compiled in place against the HIP-on-CPU shim, one
+    device; its stdout is recorded in tests/golden/distFFT_ref_stdout.json by tests/golden/make_ref_samples.py) and this repo's
+    driver/distFFT.cpp (against the fake CUDA runtime) are run with the same arguments: with every number replaced by '#', the
+    reference's stdout must be, line for line and in order, a subsequence of ours (ours adds lines after the report block)."""
+    import json
     import re
-    sys.path.insert(0, ROOT)
-    from oracle import build_ref3d
-    ref_exe = os.path.join(ROOT, "oracle", "_ref", "distFFT_ref")
-    if build_ref3d() is None or not os.path.exists(ref_exe):
-        pytest.skip("oracle/_ref/distFFT_ref not built and /root/reference absent")
+    with open(os.path.join(ROOT, "tests", "golden", "distFFT_ref_stdout.json")) as f:
+        theirs = json.load(f)
     exe = tmp_path / "distFFT_fake"
     subprocess.run(["g++", "-O1", "-std=c++17", "-I", os.path.join(ROOT, "include"), "-I", "/usr/local/cuda/include", DRIVER_SRC, "-o", str(exe),
                     fake_lib, "-Wl,-rpath," + os.path.dirname(fake_lib), "-lpthread"], check=True)
-    args = ["16", "16", "16", "1"]
-    ours = subprocess.run([str(exe)] + args, capture_output=True, text=True, timeout=60, env=dict(os.environ, FAKECUDA_DEVICES="8"))
-    theirs = subprocess.run([ref_exe] + args, capture_output=True, text=True, timeout=120)
-    assert ours.returncode == 0 and theirs.returncode == 0, ours.stderr + theirs.stderr
+    ours = subprocess.run([str(exe)] + theirs["args"], capture_output=True, text=True, timeout=60, env=dict(os.environ, FAKECUDA_DEVICES="8"))
+    assert ours.returncode == 0 and theirs["returncode"] == 0, ours.stderr
 
     def shape(text):
         out = []
@@ -230,13 +226,12 @@ def test_driver_stdout_surface_is_the_reference_drivers(fake_lib, tmp_path):
             if line:
                 out.append(line)
         return out
-    a, b = shape(theirs.stdout), shape(ours.stdout)
+    a, b = shape(theirs["stdout"]), shape(ours.stdout)
     assert "Size: #x#x#" in a and "Max error: #" in a and a.count("t#: #, t#: #, t#: #, t#: #, total: #") == 4
     it = iter(b)
     missing = [line for line in a if line not in it]          # `in` consumes the iterator: an ordered-subsequence check
     assert not missing, (missing, b)
     # the reference's argument check (fftSpeed3d_c2c.cpp:28-31)
-    bad = subprocess.run([ref_exe, "16", "16"], capture_output=True, text=True, timeout=60)
-    ours_bad = subprocess.run([str(exe), "16", "16"], capture_output=True, text=True, timeout=60)
-    assert bad.returncode != 0 and ours_bad.returncode != 0
-    assert [l for l in bad.stdout.splitlines() if "format of arguments" in l] == [l for l in ours_bad.stdout.splitlines() if "format of arguments" in l] != []
+    ours_bad = subprocess.run([str(exe)] + theirs["bad_args"], capture_output=True, text=True, timeout=60)
+    assert theirs["bad_args_returncode"] != 0 and ours_bad.returncode != 0
+    assert [l for l in theirs["bad_args_stdout"].splitlines() if "format of arguments" in l] == [l for l in ours_bad.stdout.splitlines() if "format of arguments" in l] != []
