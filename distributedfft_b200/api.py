@@ -37,7 +37,7 @@ __all__ = [
     "EXCHANGE_NCCL", "EXCHANGE_STAGED", "SCALE_BACKWARD", "NO_FUSE", "FORCE_FUSE", "OVERLAP_X", "NATURAL_SPECTRUM", "DRY_RUN", "NO_PIPELINE", "NO_TMA", "FORCE_PIPELINE", "DfftError", "lib", "LIB_PATH", "Plan", "LocalComm",
     "BootstrapComm", "fft_mpi_init", "fft_mpi_plan_dft_c2c_3d", "fft_mpi_execute_dft_3d_c2c", "fft_mpi_destroy_plan",
     "fft_mpi_alloc_local_memory", "fft_mpi_local_size_3d", "fft_mpi_cleanup", "getMaxDataCount", "supported_lengths",
-    "fft_lines", "lines_ops", "LinesPlan", "length_kind", "length_schedule", "memcpy_htod", "memcpy_dtoh", "exchange_table", "comm_allgather",
+    "fft_lines", "lines_ops", "LinesPlan", "length_kind", "length_schedule", "fused_kinds", "memcpy_htod", "memcpy_dtoh", "exchange_table", "comm_allgather",
 ]
 
 
@@ -102,6 +102,7 @@ def lib():
     L.dfft_debug_lines_ops.argtypes = [i, ll, ll, ll, ll, ll, i, i, i, ctypes.c_char_p, ll]
     L.dfft_debug_lines_ops.restype = ll
     L.dfft_length_schedule.argtypes = [i, i, P(ctypes.c_int), i]
+    L.dfft_debug_fused_kinds.argtypes = [i, i]
     L.dfft_debug_fused3_order.argtypes = [ll, ll, i, i, i, i, i, ll, P(ll)]
     L.dfft_debug_fused3_order.restype = ll
     L.dfft_memcpy.argtypes = [vp, vp, ctypes.c_size_t, i]
@@ -125,6 +126,11 @@ def supported_lengths(precision=DOUBLE):
 def length_kind(n, precision=DOUBLE):
     """2 = tuned kernel, 1 = run-time-scheduled kernel (2..13-smooth lengths), 0 = unsupported."""
     return int(lib().dfft_length_kind(n, precision))
+
+
+def fused_kinds(n, precision=DOUBLE):
+    """bit mask of the multi-role kernels length n has (see dfft_debug_fused_kinds); -1 if unsupported"""
+    return int(lib().dfft_debug_fused_kinds(n, precision))
 
 
 def length_schedule(n, precision=DOUBLE):

@@ -57,6 +57,18 @@ extern "C" int dfft_length_kind(int n, int precision)
     return !e ? 0 : (e->gen ? 1 : 2);
 }
 
+/* test hook: which multi-role kernels the entry of length n has (bit k: fused t0 kind k of FusedKind, bit 4: the kernel-chain
+ * link fused_yx, bit 5: the single-kernel forward fused3); -1 if the length is unsupported */
+extern "C" int dfft_debug_fused_kinds(int n, int precision)
+{
+    if (n < 1 || n > (1 << 20) || (precision != DFFT_DOUBLE && precision != DFFT_FLOAT)) return -1;
+    const SizeEntry* e = find_size_entry(n, precision);
+    if (!e) return -1;
+    int m = 0;
+    for (int k = 0; k < FK_COUNT; k++) m |= e->fused[k] ? 1 << k : 0;
+    return m | (e->fused_yx ? 1 << 4 : 0) | (e->fused3 ? 1 << 5 : 0);
+}
+
 /* radix schedule the library uses for length n (contiguous-pass schedule for tuned lengths, the run-time schedule for
  * generic ones); returns the number of stages, 0 if unsupported */
 extern "C" int dfft_length_schedule(int n, int precision, int* radices, int max_radices)
@@ -660,7 +672,10 @@ static int plan_create(long long n0, long long n1, long long n2, void* in, void*
         // contiguous role then hides entirely under the link time); on one GPU / NCCL the two HBM-bound sweeps
         // are currently faster (profiles/: SM-side time of both roles adds up), so it is opt-in there.
         const char* env = getenv("DFFT_FUSE");
-        const bool can = n1 == n2 && ez->fused[FK_ZY] != nullptr;
+        // the fused kernel this plan would launch: the chunked kinds carry the exchange (P > 1); an entry has no launcher for a
+        // kind whose roles do not fit one CTA's shared memory (make_entry), and such a plan runs the two passes separately
+        const int kind = P > 1 ? (direction == DFFT_FORWARD ? FK_ZY_CO : FK_YZ_CI) : (direction == DFFT_FORWARD ? FK_ZY : FK_YZ);
+        const bool can = n1 == n2 && ez->fused[kind] != nullptr;
         bool want = P > 1 && xmode == DFFT_EXCHANGE_P2P;
         if (env) want = strcmp(env, "0") != 0;
         if (flags & DFFT_FORCE_FUSE) want = true;

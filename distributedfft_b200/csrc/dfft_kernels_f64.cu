@@ -20,7 +20,9 @@ void register_f64(std::vector<SizeEntry>& v)
     v.push_back(make_entry<T, Cfg<Sched<2048, 16, 16, 16, 8>, 1, false, 4, false>, Cfg<Sched<2048, 16, 16, 16, 8>, 4, false, 1, false>>());
     v.push_back(make_entry<T, Cfg<Sched<4096, 16, 16, 16, 16>, 1, false, 2, false>, Cfg<Sched<4096, 16, 16, 16, 16>, 2, false, 1, false>>());
 #ifdef DFFT_EXPERIMENTS   // build with -DDFFT_EXPERIMENTS (python -m distributedfft_b200.build --experiments): alternate tunings selected
-                          // at run time with DFFT_VARIANT=n; the default library ships only configurations that passed parity on hardware
+                          // at run time with DFFT_VARIANT=n; every instantiation of the default tables runs against an fp64 reference
+                          // in tests/test_gpu_parity.py / test_gpu_multi.py (cases: tests/kernel_matrix.py, completeness checked on
+                          // the CPU by tests/test_kernel_matrix_complete.py)
     // experiments for the fused t0 kernel (DFFT_VARIANT=1|2, not used by default): the strided role reads its tile from L2,
     // not HBM, so narrow tiles (64- / 32-byte rows) cost no DRAM efficiency there and allow 3-5 smaller CTAs per SM
     // (finer-grained phases; the fused kernel's top stall is the CTA barrier, profiles/r1_ncu_full_fused_t0_512.txt)

@@ -34,14 +34,24 @@ cudaError_t launch_pass(const void* vargs, int sm_count, cudaStream_t st)
     return cudaGetLastError();
 }
 
+// dynamic shared memory one CTA may use on sm_100 (cudaDevAttrMaxSharedMemoryPerBlockOptin: 227 KB)
+constexpr size_t DFFT_MAX_SMEM = 227 * 1024;
+// shared memory of a kernel running several TileOp roles: one exchange buffer (the largest) + every role's own part
+template <class A, class... More> constexpr size_t roles_smem()
+{
+    size_t exch = A::SM::exch_bytes, aux = A::aux_bytes;
+    ((exch = More::SM::exch_bytes > exch ? More::SM::exch_bytes : exch), ...);
+    ((aux += More::aux_bytes), ...);
+    return exch + aux;
+}
+
 template <class OpA, class OpB, typename T, int MINB>
 cudaError_t launch_fused(const void* va, const void* vb, const FusedCtl* ctl, int sm_count, cudaStream_t st)
 {
     const TileArgs<T>& a = *reinterpret_cast<const TileArgs<T>*>(va);
     const TileArgs<T>& b = *reinterpret_cast<const TileArgs<T>*>(vb);
     auto kern = fft_fused2_kernel<OpA, OpB, T, MINB>;
-    constexpr size_t exch = OpA::SM::exch_bytes > OpB::SM::exch_bytes ? OpA::SM::exch_bytes : OpB::SM::exch_bytes;
-    constexpr size_t smem = exch + OpA::aux_bytes + OpB::aux_bytes;
+    constexpr size_t smem = roles_smem<OpA, OpB>();
     static std::atomic<int> occ_cache[64];
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -72,8 +82,7 @@ cudaError_t launch_fused_yx(const void* va, const void* vb, const YxCtl* ctl, in
     const TileArgs<T>& a = *reinterpret_cast<const TileArgs<T>*>(va);
     const TileArgs<T>& b = *reinterpret_cast<const TileArgs<T>*>(vb);
     auto kern = fft_fused_yx_kernel<OpA, OpB, T, MINB>;
-    constexpr size_t exch = OpA::SM::exch_bytes > OpB::SM::exch_bytes ? OpA::SM::exch_bytes : OpB::SM::exch_bytes;
-    constexpr size_t smem = exch + OpA::aux_bytes + OpB::aux_bytes;
+    constexpr size_t smem = roles_smem<OpA, OpB>();
     static std::atomic<int> occ_cache[64];
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -102,9 +111,7 @@ cudaError_t launch_fused3(const void* va, const void* vb, const void* vc, const 
     const TileArgs<T>& b = *reinterpret_cast<const TileArgs<T>*>(vb);
     const TileArgs<T>& c = *reinterpret_cast<const TileArgs<T>*>(vc);
     auto kern = fft_fused3_kernel<OpA, OpB, OpC, T, MINB>;
-    constexpr size_t e1 = OpA::SM::exch_bytes > OpB::SM::exch_bytes ? OpA::SM::exch_bytes : OpB::SM::exch_bytes;
-    constexpr size_t exch = e1 > OpC::SM::exch_bytes ? e1 : OpC::SM::exch_bytes;
-    constexpr size_t smem = exch + OpA::aux_bytes + OpB::aux_bytes + OpC::aux_bytes;
+    constexpr size_t smem = roles_smem<OpA, OpB, OpC>();
     static std::atomic<int> occ_cache[64];
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -190,16 +197,22 @@ SizeEntry make_entry(int variant = 0)
     using OY2 = TileOp<SS, T, Y::C, MAP_C, MAP_C, false, false, false, false, false, H1, H1>;
     using OYco = TileOp<SS, T, PEER::C, MAP_C, MAP_C, false, false, true, false, false, H1, 0>;
     using OYci = TileOp<SS, T, Y::C, MAP_C, MAP_C, false, true, false, false, false, H1, H2>;
-    e.fused[FK_ZY] = launch_fused<OZ, OY2, T, Y::MB>;
-    e.fused[FK_ZY_CO] = launch_fused<OZp, OYco, T, PEER::MB>;
-    e.fused[FK_YZ] = launch_fused<OY, OZ2, T, Y::MB>;
-    e.fused[FK_YZ_CI] = launch_fused<OYci, OZ2, T, Y::MB>;
+    // a multi-role kernel whose roles together need more shared memory than one CTA may have cannot launch: it gets no
+    // launcher (nullptr), and plans of this length run the passes as separate kernels instead
+    if constexpr (roles_smem<OZ, OY2>() <= DFFT_MAX_SMEM) e.fused[FK_ZY] = launch_fused<OZ, OY2, T, Y::MB>;
+    if constexpr (roles_smem<OZp, OYco>() <= DFFT_MAX_SMEM) e.fused[FK_ZY_CO] = launch_fused<OZp, OYco, T, PEER::MB>;
+    if constexpr (roles_smem<OY, OZ2>() <= DFFT_MAX_SMEM) e.fused[FK_YZ] = launch_fused<OY, OZ2, T, Y::MB>;
+    if constexpr (roles_smem<OYci, OZ2>() <= DFFT_MAX_SMEM) e.fused[FK_YZ_CI] = launch_fused<OYci, OZ2, T, Y::MB>;
     // whole forward transform of a device in one kernel: needs the X role to fill the peer-store CTA shape
+    e.fused3 = nullptr;
+    e.fused_yx = nullptr;
     if constexpr (XS::T * X::C == NTP) {
         using OX = TileOp<XS, T, X::C, MAP_C, MAP_T, false, false, false, false>;
-        e.fused3 = launch_fused3<OZp, OYco, OX, T, (PEER::MB < X::MB ? PEER::MB : X::MB)>;
-        e.fused_yx = launch_fused_yx<OYco, OX, T, (PEER::MB < X::MB ? PEER::MB : X::MB)>;
-    } else { e.fused3 = nullptr; e.fused_yx = nullptr; }
+        if constexpr (roles_smem<OZp, OYco, OX>() <= DFFT_MAX_SMEM)
+            e.fused3 = launch_fused3<OZp, OYco, OX, T, (PEER::MB < X::MB ? PEER::MB : X::MB)>;
+        if constexpr (roles_smem<OYco, OX>() <= DFFT_MAX_SMEM)
+            e.fused_yx = launch_fused_yx<OYco, OX, T, (PEER::MB < X::MB ? PEER::MB : X::MB)>;
+    }
     return e;
 }
 

@@ -111,12 +111,17 @@ const TmaEntry* find_tma_entry(int N, int prec)
     if (env && atoi(env) == 0) return nullptr;
     if (getenv("DFFT_GENERIC") && atoi(getenv("DFFT_GENERIC")) != 0) return nullptr;
     if (!tma_available()) return nullptr;
-    static thread_local TmaEntry forced;
-    for (const TmaEntry& e : tma_table())
-        if (e.N == N && e.prec == prec) {
-            if (env && atoi(env) == 2) { forced = e; forced.use = 0xf; return &forced; }
-            return &e;
-        }
+    // DFFT_TMA=2: a copy of every entry with all modes on.  One copy per entry, built once: a plan keeps the pointers of all
+    // three axes (and of other plans) alive, so they must not share one slot.
+    static std::vector<TmaEntry> forced;
+    static std::once_flag once;
+    std::call_once(once, [] {
+        forced = tma_table();
+        for (TmaEntry& e : forced) e.use = 0xf;
+    });
+    const std::vector<TmaEntry>& t = env && atoi(env) == 2 ? forced : tma_table();
+    for (const TmaEntry& e : t)
+        if (e.N == N && e.prec == prec) return &e;
     return nullptr;
 }
 

@@ -96,6 +96,10 @@ int dfft_version(void);
  * 12800 in float, i.e. while two copies of a line fit in shared memory); 0: unsupported (other primes, or longer:
  * the reference switches to multi-upload passes there, templateFFT.cpp:4007-4106, which this library does not have) */
 int dfft_length_kind(int n, int precision);
+/* test hook (host only): the multi-role kernels the table entry of length n has -- bit k: fused t0 kind k (0 Z+Y, 1 Z+Y with
+ * the chunked store, 2 Y+Z, 3 Y+Z with the chunked load), bit 4: the kernel-chain link, bit 5: the single-kernel forward.  A
+ * kind whose roles need more shared memory than one CTA may have is absent; -1: unsupported length */
+int dfft_debug_fused_kinds(int n, int precision);
 /* radix schedule used for length n (stage order as executed); returns the number of stages, 0 if unsupported */
 int dfft_length_schedule(int n, int precision, int* radices, int max_radices);
 /* test hook (host only): ticket order of the single-kernel forward path (fft_fused3_kernel); out = role (0 Z, 1 Y, 2 X),

@@ -1,13 +1,15 @@
 """Helpers for the -m gpu parity tests: drive libdfft.so through its C ABI (via the ctypes
 binding) on torch-allocated device buffers, one host thread per device like the reference driver
 (3dmpifft_opt/fftSpeed3d_c2c.cpp:49-51)."""
+import functools
 import threading
 
 import numpy as np
 import torch
 
 import distributedfft_b200 as dfft
-from oracle import SlabGeometry
+import kernel_matrix as km
+from oracle import NumpySlab, SlabGeometry
 
 CDT = {dfft.DOUBLE: (np.complex128, torch.complex128), dfft.FLOAT: (np.complex64, torch.complex64)}
 
@@ -57,6 +59,8 @@ def run_slab(n0, n1, n2, P, direction, inputs, precision=dfft.DOUBLE, flags=0, r
                 out["launches"] = plan.launches
                 out["exchange"] = plan.exchange
                 out["fused"] = plan.fused
+                out["tma_mask"] = plan.tma_mask
+                out["pipeline_chain"] = plan.pipeline_chain
             out["buf1"] = fetch(plan.bufferDev1, mc)
             out["buf2"] = fetch(plan.bufferDev2, mc)
             out["counts"] = (plan.in_count, plan.out_count, plan.maxDataCountInDevice)
@@ -77,3 +81,61 @@ def run_slab(n0, n1, n2, P, direction, inputs, precision=dfft.DOUBLE, flags=0, r
     if errs:
         raise RuntimeError("device thread failed:\n" + "\n".join(e for _, e in errs))
     return res
+
+
+@functools.lru_cache(maxsize=1)
+def matrix_data(shape, precision):
+    """seeded standard-normal complex input A [x][y][z] and backward input B [y][z][x], both rounded to `precision`, and
+    their fp64 references: the forward spectrum of A laid out [y][z][x], the unnormalised inverse of B laid out [x][y][z]"""
+    n0, n1, n2 = shape
+    npdt = CDT[precision][0]
+    rng = np.random.default_rng([n0, n1, n2, precision])
+    A = (rng.standard_normal(shape) + 1j * rng.standard_normal(shape)).astype(npdt)
+    B = (rng.standard_normal((n1, n2, n0)) + 1j * rng.standard_normal((n1, n2, n0))).astype(npdt)
+    ref_f = np.ascontiguousarray(np.fft.fftn(A.astype(np.complex128)).transpose(1, 2, 0))
+    ref_b = np.fft.ifftn(B.astype(np.complex128).transpose(2, 0, 1)) * (n0 * n1 * n2)
+    return A, B, ref_f, ref_b
+
+
+def run_matrix_case(case):
+    """one kernel_matrix case on case.P devices against the fp64 reference (environment already set): forward, backward
+    and the scaled round trip, per device over its slab; every plan must have taken the path the case names"""
+    n0, n1, n2 = case.shape
+    N = n0 * n1 * n2
+    P = case.P
+    g = SlabGeometry(n0, n1, n2, P)
+    A, B, ref_f, ref_b = matrix_data(case.shape, case.precision)
+
+    def expect(res, direction):
+        for r in res:
+            for k, _ in case.expect:
+                v = km.expected(case, k, direction)
+                if k == "pipeline_chain" and direction != dfft.FORWARD:
+                    continue
+                assert r[k] == v, (case.id, direction, k, r[k], v)
+
+    fwd = None
+    if dfft.FORWARD in case.directions:
+        fwd = run_slab(n0, n1, n2, P, dfft.FORWARD, NumpySlab(n0, n1, n2, P).scatter_input(A), case.precision, case.flags)
+        expect(fwd, dfft.FORWARD)
+        for q in range(P):
+            want = ref_f[q * g.yd: q * g.yd + g.n1l(q)]
+            km.check(fwd[q]["buf2"][: g.out_count(q)], want, case.precision, N, f"{case.id} forward device {q}")
+    if dfft.BACKWARD in case.directions:
+        ins = []
+        for q in range(P):
+            b = np.zeros(g.max_count(q), dtype=B.dtype)
+            blk = B[q * g.yd: q * g.yd + g.n1l(q)].reshape(-1)
+            b[: blk.size] = blk
+            ins.append(b)
+        bwd = run_slab(n0, n1, n2, P, dfft.BACKWARD, ins, case.precision, case.flags)
+        expect(bwd, dfft.BACKWARD)
+        for p in range(P):
+            want = ref_b[p * g.xd: p * g.xd + g.n0l(p)]
+            km.check(bwd[p]["buf2"][: g.in_count(p)], want, case.precision, N, f"{case.id} backward device {p}")
+        if fwd is not None:
+            rt = run_slab(n0, n1, n2, P, dfft.BACKWARD, [r["buf2"] for r in fwd], case.precision, case.flags | dfft.SCALE_BACKWARD)
+            expect(rt, dfft.BACKWARD)
+            for p in range(P):
+                want = A[p * g.xd: p * g.xd + g.n0l(p)]
+                km.check(rt[p]["buf2"][: g.in_count(p)], want, case.precision, N, f"{case.id} scaled round trip device {p}")

@@ -230,3 +230,26 @@ def test_overlapped_forward_matches_default_path(P, n):
     for p in range(P):
         assert b[p]["launches"] < a[p]["launches"]
         assert np.array_equal(a[p]["buf2"], b[p]["buf2"]), p
+
+
+# ---- the instantiation matrix on two devices (tests/kernel_matrix.py): chunked kinds, chunked fused t0, the kernel chain -----
+import kernel_matrix as km  # noqa: E402
+from gpu_helpers import run_matrix_case  # noqa: E402
+
+MATRIX_2 = km.two_device_cases()
+
+
+@pytest.mark.parametrize("case", MATRIX_2, ids=[c.id for c in MATRIX_2])
+def test_kernel_matrix_two_devices(case, monkeypatch):
+    """Two-device cases of the matrix (odd lengths split unevenly): forward and backward per device against numpy's fftn in
+    complex128, max|err| / rms(ref) <= 1e-13 log2 N (fp64) / 1e-6 log2 N (fp32), the scaled round trip, and the plan's path
+    (fused, kernel chain, exchange)."""
+    need(case.P)
+    for k, v in case.env:
+        monkeypatch.setenv(k, v)
+    run_matrix_case(case)
+
+
+def test_kernel_matrix_error_report():
+    """prints the worst error / bound per precision of the matrix cases that ran in this session (no assertion)"""
+    print("\nkernel matrix:", km.report() or "no case ran")

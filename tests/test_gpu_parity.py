@@ -432,3 +432,41 @@ def test_natural_order_spectrum_single_device(n0, n1, n2):
     assert np.abs(f[0]["buf2"] - ref).max() <= 1e-12 * np.log2(A.size) * np.abs(ref).max()
     b = run_slab(n0, n1, n2, 1, BACKWARD, [ref], flags=dfft.NATURAL_SPECTRUM)
     assert np.abs(b[0]["buf2"] / A.size - A.reshape(-1)).max() <= 1e-11
+
+
+# ---- the instantiation matrix (tests/kernel_matrix.py): every kernel the library ships, against an fp64 reference ----------
+import kernel_matrix as km  # noqa: E402
+from gpu_helpers import run_matrix_case  # noqa: E402
+
+MATRIX_1 = km.single_device_cases()
+
+
+@pytest.mark.parametrize("case", MATRIX_1, ids=[c.id for c in MATRIX_1])
+def test_kernel_matrix_single_device(case, monkeypatch):
+    """One tuned length (or generic / TMA configuration) per case: forward and backward against numpy's fftn in complex128 of the
+    same rounded input, max|err| / rms(ref) <= 1e-13 log2 N (fp64) / 1e-6 log2 N (fp32), plus the SCALE_BACKWARD round trip; the
+    plan must report the path the case names (fused, TMA mask)."""
+    for k, v in case.env:
+        monkeypatch.setenv(k, v)
+    run_matrix_case(case)
+
+
+FOUR_STEP_CASES = [(p, first, n) for p in (km.D, km.F) for t in (km.FOUR_STEP[p], km.FOUR_STEP_GENERIC[p]) for first, n in t.items()]
+
+
+@pytest.mark.parametrize("precision,first,n", FOUR_STEP_CASES, ids=[f"{km.PREC_NAME[p]}-{n}-first{f}" for p, f, n in FOUR_STEP_CASES])
+def test_kernel_matrix_four_step(precision, first, n):
+    """Long lines through the four-step plan, whose first pass (PK_XF_TW of the first factor) runs every tuned length."""
+    nl = km.four_step_lines(n)
+    rng = np.random.default_rng(n)
+    a = (rng.standard_normal((nl, n)) + 1j * rng.standard_normal((nl, n))).astype(CDT[precision][0])
+    plan = dfft.LinesPlan(n, 1, nl, nl, n, 0, precision)
+    try:
+        for direction in (FORWARD, BACKWARD):
+            ref = np.fft.fft(a.astype(np.complex128), axis=1) if direction == FORWARD else np.fft.ifft(a.astype(np.complex128), axis=1) * n
+            t = _dev_array(a.reshape(-1), precision)
+            plan.execute(t.data_ptr(), direction)
+            plan.synchronize()
+            km.check(t.cpu().numpy(), ref, precision, n, f"four-step {n} = {first} x {n // first} direction {direction}")
+    finally:
+        plan.destroy()
